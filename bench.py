@@ -20,6 +20,10 @@ A "step" is one pass of the hot path over one batch of synthetic input: BASELINE
          (pipelined; the un-pipelined step is reported too); c5 = configs[4] on spatial map shards (strong scaling).
   --impl reference   the reference's own CPU path (oracle/_ref = its compiled ODE when present, else the C port)
          on all host threads, on a bounded sample of the same workload per step.
+  --dump-outputs DIR  after the timed steps, what the last timed step returned as DIR/<name>.npy (float32 / float64,
+         exact): valid (verdict bytes), valid_bits (bit-packed verdicts, uint32 words), valid_index (ordered indices of the
+         valid samples), valid_count; N > 1: all_valid_bits (the all-gathered masks), written by rank 0. --impl
+         reference: valid of its sample. The inputs are seeded, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -107,6 +111,15 @@ def make_inputs(rank: int, n: int, workload: str = "c2", world: int = 1):
     m = synth.make_fbm_map(MAP_N, MAP_N, MAP_RES, seed=MAP_SEED, amp=0.6)
     poses = synth.make_terrain_poses(m, n, seed=POSE_SEED, start=rank * n)
     return m, poses
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: one <name>.npy per output array; the integer outputs are written as float64 (exact)."""
+    os.makedirs(path, exist_ok=True)
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), name
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def cpu_oracle(params):
@@ -281,8 +294,10 @@ def run_reference(args):
         o.check_poses_mt(poses[:20000], cores)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        o.check_poses_mt(poses, cores)
+        valid = o.check_poses_mt(poses, cores)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"valid": valid.astype(np.float32)})
     value = sample_n * args.steps / dt
     sample = (f"first {sample_n} poses of the 1M-pose workload per step, {cores} threads (best of a probe over "
               f"8..{os.cpu_count()} threads), one ODE world per thread")
@@ -305,7 +320,10 @@ def main():
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--workload", default="c2", choices=["c2", "c5"],
                     help="c2 = BASELINE configs[1] (default, the metric's config); c5 = configs[4], 4000x4000 map, spatial slabs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -430,6 +448,15 @@ def main():
     wall = time.perf_counter() - wall0
     dev_ms = sum(s.elapsed_time(e) for s, e in ev)
     launches = chk.stats()["kernel_launches"] - launches0      # kernels of this library launched inside the timed region
+    if args.dump_outputs and rank == 0:    # the last timed step's outputs, before the passes below overwrite them
+        cnt = int(loc_cnt.item())
+        outs = {"valid": d_valid.cpu().numpy().astype(np.float32),
+                "valid_bits": my_bits[(args.steps - 1) & 1].cpu().numpy().view(np.uint32).astype(np.float64),
+                "valid_index": loc_idx[:cnt].cpu().numpy().astype(np.float64),
+                "valid_count": np.array([cnt], np.float64)}
+        if world > 1:
+            outs["all_valid_bits"] = all_bits.cpu().numpy().view(np.uint32).astype(np.float64)
+        dump_outputs(args.dump_outputs, outs)
     # second pass, per-stage timing ON (the stages of a round then run one after the other on the call's stream): stage
     # durations from the library's CUDA events, and the throughput of that serial order
     chk.setTiming(True)

@@ -1,6 +1,7 @@
 """Generate tests/golden/*.npz with the reference's own compiled ODE (oracle/_ref/liborc_ref.so).
 
-Run in the build container (needs /root/reference):  python oracle/make_golden.py
+Needs the reference's sources (REF of oracle/Makefile):  python oracle/make_golden.py [fresh]
+(`fresh` rewrites only tests/golden/reference_fresh.npz.)
 Inputs are regenerated from seeds by tests/cases.py; the fixtures hold only the packed result masks plus a
 checksum of the inputs (so generator drift is detected) -- a few KB each.
 """
@@ -89,7 +90,35 @@ def main() -> None:
     path = os.path.join(ROOT, "tests", "golden", "reference_masks.npz")
     np.savez_compressed(path, **out)
     print("wrote", path, os.path.getsize(path), "bytes")
+    fresh(maps)
+
+
+def fresh(maps) -> None:
+    """tests/golden/reference_fresh.npz: pose and box verdicts of cases.FRESH_CASES."""
+    from art_planner_b200 import synth
+    out = {}
+    for name, mk, n_p, p_seed, n_b, b_seed, tilt, zr in cases.FRESH_CASES:
+        m = maps[mk]
+        o = Oracle(cases.PARAMS["yaml"], "reference")
+        o.set_map(m)
+        poses = synth.make_terrain_poses(m, n_p, seed=p_seed)
+        v = o.check_poses(poses)
+        out[name + "/mask"] = np.packbits(v)
+        out[name + "/sha"] = np.array(digest(m.elevation, m.elevation_masked, poses))
+        for which in (0, 1):
+            org, rot = cases.box_samples(m, n_b, b_seed, which, tilt, zr)
+            hit = o.box_collide(which, org, rot)
+            out[f"{name}/{which}/mask"] = np.packbits(hit)
+            out[f"{name}/{which}/sha"] = np.array(digest(m.elevation, m.elevation_masked, org, rot))
+        print(f"{name}: valid={int(v.sum())}/{n_p}")
+    path = os.path.join(ROOT, "tests", "golden", "reference_fresh.npz")
+    np.savez_compressed(path, **out)
+    print("wrote", path, os.path.getsize(path), "bytes")
 
 
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] == ["fresh"]:
+        build("ref")
+        fresh({k: f() for k, f in cases.MAPS.items()})
+    else:
+        main()

@@ -167,6 +167,17 @@ BOX_CASES = [
 ]
 BOX_N = 20000
 
+# Port vs compiled reference on seeds no other case uses and on the adversarial maps, pose and box level (yaml geometry;
+# golden: tests/golden/reference_fresh.npz): (name, map, n poses, pose seed, n boxes, box seed, tilt, zr)
+FRESH_CASES = [
+    ("fresh_fixture", "fixture", 5000, 1234, 5000, 4321, 0.8, 0.4),
+    ("fresh_ramp", "ramp", 5000, 1234, 5000, 4321, 0.8, 0.4),
+    ("fresh_fbm_rough", "fbm_rough", 5000, 1234, 5000, 4321, 0.8, 0.4),
+    ("adversarial_terraces", "terraces", 20000, 31, 20000, 99, 0.9, 0.35),
+    ("adversarial_spikes", "spikes", 20000, 31, 20000, 99, 0.9, 0.35),
+    ("adversarial_terraces_tilted", "terraces_tilted", 20000, 31, 20000, 99, 0.9, 0.35),
+]
+
 # (name, map, params, n_edges, n_steps, seed)
 # addValidMilestone connection batches (prm_motion_cost.cpp:341-372): (name, map, params, n, seed, dmin, dmax);
 # n_interp = (unsigned)(lateralDistance / 0.5) per edge -> 0..6 interior states here

@@ -26,6 +26,18 @@ def test_reference_arm_json_line():
     assert "workload" in d["config"]
 
 
+def test_reference_arm_dumps_its_outputs(tmp_path):
+    """--dump-outputs writes the verdicts of the last timed step as float .npy files, identical from run to run."""
+    import numpy as np
+    for d in ("a", "b"):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2", "--warmup", "1",
+                            "--dump-outputs", str(tmp_path / d)], capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert r.returncode == 0, r.stderr[-2000:]
+    a, b = (np.load(tmp_path / d / "valid.npy") for d in ("a", "b"))
+    assert a.dtype == np.float32 and a.shape == (200_000,) and 0 < a.sum() < len(a)
+    assert np.array_equal(a, b)
+
+
 def test_bench_metric_matches_baseline_json():
     b = json.load(open(os.path.join(ROOT, "BASELINE.json")))
     src = open(os.path.join(ROOT, "bench.py")).read()

@@ -1,5 +1,5 @@
 """CPU-only: the oracle restatement (oracle/artp_oracle.c) against the golden masks produced by the reference's
-own compiled ODE, and -- where /root/reference exists -- against that compiled library directly."""
+own compiled ODE (oracle/make_golden.py)."""
 import hashlib
 import os
 
@@ -93,39 +93,41 @@ def test_empty_batches(maps, port_lib):
     assert o.check_poses(np.zeros((0, 7))).shape == (0,)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/ode"), reason="reference tree not present on this box")
-def test_port_equals_compiled_reference_on_fresh_seeds(maps, port_lib):
-    """Fresh seeds (not in the golden file): port == compiled reference ODE, pose and box level."""
-    port_lib.build("ref")
-    for mk in ("fixture", "ramp", "fbm_rough"):
-        m = maps(mk)
-        P = port_lib.Oracle(cases.PARAMS["yaml"], "port")
-        R = port_lib.Oracle(cases.PARAMS["yaml"], "reference")
-        P.set_map(m)
-        R.set_map(m)
-        poses = synth.make_terrain_poses(m, 5000, seed=1234)
-        assert np.array_equal(P.check_poses(poses), R.check_poses(poses))
-        for which in (0, 1):
-            org, rot = cases.box_samples(m, 5000, 4321, which, 0.8, 0.4)
-            assert np.array_equal(P.box_collide(which, org, rot), R.box_collide(which, org, rot))
+@pytest.fixture(scope="module")
+def fresh():
+    return np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_fresh.npz"))
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/ode"), reason="reference tree not present on this box")
-@pytest.mark.parametrize("mk", [cases.terraces, cases.spikes, cases.terraces_tilted], ids=["terraces", "spikes", "terraces_tilted"])
-def test_port_equals_compiled_reference_on_adversarial_maps(mk, port_lib):
-    port_lib.build("ref")
-    m = mk()
+def port_equals_compiled_reference(case, maps, port_lib, fresh):
+    """Port pose and box verdicts == the compiled reference ODE's (stored by oracle/make_golden.py); returns the
+    pose verdicts."""
+    name, mk, n_p, p_seed, n_b, b_seed, tilt, zr = case
+    m = maps(mk)
     P = port_lib.Oracle(cases.PARAMS["yaml"], "port")
-    R = port_lib.Oracle(cases.PARAMS["yaml"], "reference")
     P.set_map(m)
-    R.set_map(m)
-    poses = synth.make_terrain_poses(m, 20000, seed=31)
+    poses = synth.make_terrain_poses(m, n_p, seed=p_seed)
+    assert digest(m.elevation, m.elevation_masked, poses) == str(fresh[name + "/sha"]), "generator drift"
     a = P.check_poses(poses)
-    assert 0 < a.sum() < len(a)
-    assert np.array_equal(a, R.check_poses(poses))
+    assert np.array_equal(a, unpack(fresh, name + "/mask", n_p))
     for which in (0, 1):
-        org, rot = cases.box_samples(m, 20000, 99, which, 0.9, 0.35)
-        assert np.array_equal(P.box_collide(which, org, rot), R.box_collide(which, org, rot))
+        org, rot = cases.box_samples(m, n_b, b_seed, which, tilt, zr)
+        assert digest(m.elevation, m.elevation_masked, org, rot) == str(fresh[f"{name}/{which}/sha"])
+        assert np.array_equal(P.box_collide(which, org, rot), unpack(fresh, f"{name}/{which}/mask", n_b))
+    return a
+
+
+def test_port_equals_compiled_reference_on_fresh_seeds(maps, port_lib, fresh):
+    """Fresh seeds (not in reference_masks.npz): port == compiled reference ODE, pose and box level."""
+    for case in cases.FRESH_CASES:
+        if case[0].startswith("fresh_"):
+            port_equals_compiled_reference(case, maps, port_lib, fresh)
+
+
+@pytest.mark.parametrize("mk", ["terraces", "spikes", "terraces_tilted"])
+def test_port_equals_compiled_reference_on_adversarial_maps(mk, maps, port_lib, fresh):
+    case = next(c for c in cases.FRESH_CASES if c[0] == "adversarial_" + mk)
+    a = port_equals_compiled_reference(case, maps, port_lib, fresh)
+    assert 0 < a.sum() < len(a)
 
 
 def test_hard_regime_exit_mix(maps, port_lib):

@@ -11,7 +11,7 @@ LIB = os.path.join(HERE, "libartp.so")
 # the motion-cost network does not.
 SOURCES = [("artp_capi.cu", ["-fmad=false", "-Xcompiler", "-fPIC,-ffp-contract=off"]),
            ("artp_cnn.cu", ["-Xcompiler", "-fPIC"])]
-HEADERS = ["artp_device.cuh", "artp_kernels.cuh", "artp_sampler.cuh", "artp_tiles.cuh", "artp_basic.cuh", "artp_cnn.h", os.path.join("..", "..", "include", "artp.h")]
+HEADERS = ["artp_device.cuh", "artp_kernels.cuh", "artp_sampler.cuh", "artp_tiles.cuh", "artp_basic.cuh", "artp_roadmap.cuh", "artp_cnn.h", os.path.join("..", "..", "include", "artp.h")]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17"]
 

@@ -44,6 +44,11 @@ class ArtpBasicParams(C.Structure):
         "foothold_margin_min_step", "foothold_size")]
 
 
+class ArtpGrid(C.Structure):
+    _fields_ = [("elevation", C.c_void_p), ("traversability_thresholded", C.c_void_p), ("rows", C.c_int), ("cols", C.c_int),
+                ("res", C.c_double), ("cx", C.c_double), ("cy", C.c_double)]
+
+
 class ArtpStats(C.Structure):
     _fields_ = [("poses_checked", C.c_uint64), ("poses_deferred", C.c_uint64), ("kernel_launches", C.c_uint64),
                 ("last_deferred", C.c_uint32), ("last_launches", C.c_uint32), ("last_queued_boxes", C.c_uint32),
@@ -111,6 +116,10 @@ def load():
     lib.artp_set_timing.argtypes = [vp, i32]
     lib.artp_get_last_timing.argtypes = [vp, C.POINTER(C.c_float)]
     lib.artp_get_last_stage_timing.argtypes = [vp, C.POINTER(C.c_float)]
+    lib.artp_compute_change.argtypes = [vp, C.POINTER(ArtpGrid), C.POINTER(ArtpGrid), C.c_float, vp]
+    lib.artp_compute_change_device.argtypes = [vp, C.POINTER(ArtpGrid), C.POINTER(ArtpGrid), C.c_float, vp, vp]
+    lib.artp_roadmap_updates.argtypes = [vp, vp, sz, vp, sz, vp, vp]
+    lib.artp_roadmap_updates_device.argtypes = [vp, vp, sz, vp, sz, vp, vp, vp]
     lib.artp_version.restype = C.c_char_p
     lib.artp_cost_weights_size.restype = C.c_size_t
     lib.artp_set_cost_weights.argtypes = [vp, vp, sz]

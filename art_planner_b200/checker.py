@@ -194,6 +194,79 @@ class StateValidityChecker:
                                                           None if row is None else row.ctypes.data))
         return (cum, row) if want_host else None
 
+    def computeChange(self, map_new, map_old, height_change_for_update: float, want_layer: bool = True, out=None):
+        """processors::computeChange (change.cpp:9-51) on the device. map_new / map_old: objects with `elevation` and
+        `traversability_thresholded` ([rows, cols], grid_map column-major), `res`, `cx`, `cy`. numpy layers go through the
+        host entry point and return the float `updated` layer of the new map (Fortran-order, exact 0 / 1; None when
+        want_layer is False). CUDA float32 torch layers -- [rows, cols] views with column-major strides, e.g. `t.t()` of a
+        contiguous [cols, rows] tensor -- go through the device entry point on torch's current stream and return the
+        layer as such a view (or fill `out`). The bit-packed layer stays on the handle for roadmapUpdates()."""
+        lib, h = self._h.lib, self._h
+        thr = float(height_change_for_update)
+        if _is_torch_cuda(map_new.elevation):
+            import torch
+            grids = []
+            for m in (map_new, map_old):
+                for a in (m.elevation, m.traversability_thresholded):
+                    assert _is_torch_cuda(a) and a.dtype == torch.float32 and a.dim() == 2 and a.t().is_contiguous()
+                assert m.elevation.shape == m.traversability_thresholded.shape
+                rows, cols = m.elevation.shape
+                grids.append(capi.ArtpGrid(m.elevation.data_ptr(), m.traversability_thresholded.data_ptr(), rows, cols,
+                                           float(m.res), float(m.cx), float(m.cy)))
+            if out is None and want_layer:
+                rows, cols = map_new.elevation.shape
+                out = torch.empty((cols, rows), dtype=torch.float32, device=map_new.elevation.device).t()
+            if out is not None:
+                assert out.shape == map_new.elevation.shape and out.t().is_contiguous()
+            h.check(lib.artp_compute_change_device(h.h, C.byref(grids[0]), C.byref(grids[1]), thr,
+                                                   None if out is None else C.c_void_p(out.data_ptr()), _stream_ptr()))
+            return out
+        keep, grids = [], []
+        for m in (map_new, map_old):
+            e = np.asfortranarray(m.elevation, dtype=np.float32)
+            t = np.asfortranarray(m.traversability_thresholded, dtype=np.float32)
+            if e.shape != t.shape:
+                raise capi.ArtpError(capi.ARTP_E_INVALID, "layer shapes differ")
+            keep += [e, t]
+            grids.append(capi.ArtpGrid(e.ctypes.data, t.ctypes.data, e.shape[0], e.shape[1], float(m.res), float(m.cx),
+                                       float(m.cy)))
+        upd = np.empty(keep[0].shape, np.float32, order="F") if want_layer else None
+        h.check(lib.artp_compute_change(h.h, C.byref(grids[0]), C.byref(grids[1]), thr,
+                                        None if upd is None else upd.ctypes.data))
+        return upd
+
+    def roadmapUpdates(self, vertex_states, edges, out_vertex=None, out_edge=None):
+        """LazyPRMStarMinUpdateMaintainer::update's per-vertex / per-edge questions (lazy_prm_star_min_update.cpp:18-91)
+        against the last computeChange() layer: vertex_states [nv, 7] float64, edges [ne, 2] (source, target) vertex
+        indices -> (vertex_flags [nv], edge_flags [ne]) uint8: 0 keep, 1 updated (-> VALIDITY_UNKNOWN), 2 outside the new
+        map (vertex removed; edge removed with it). numpy arrays use the host entry point (edges as uint32); CUDA torch
+        tensors (float64 states, int32 edges: same bits as uint32 below 2^31) the device entry point on torch's current
+        stream -- there a bad edge index is reported by pollError()."""
+        lib, h = self._h.lib, self._h
+        if _is_torch_cuda(vertex_states):
+            import torch
+            assert vertex_states.dtype == torch.float64 and vertex_states.is_contiguous() and vertex_states.shape[-1] == 7
+            assert edges.dtype == torch.int32 and edges.is_contiguous() and edges.shape[-1] == 2
+            nv, ne = vertex_states.shape[0], edges.shape[0]
+            if out_vertex is None:
+                out_vertex = torch.empty(nv, dtype=torch.uint8, device=vertex_states.device)
+            if out_edge is None:
+                out_edge = torch.empty(ne, dtype=torch.uint8, device=vertex_states.device)
+            h.check(lib.artp_roadmap_updates_device(h.h, C.c_void_p(vertex_states.data_ptr()), nv, C.c_void_p(edges.data_ptr()),
+                                                    ne, C.c_void_p(out_vertex.data_ptr()), C.c_void_p(out_edge.data_ptr()),
+                                                    _stream_ptr()))
+            return out_vertex, out_edge
+        s = np.ascontiguousarray(vertex_states, dtype=np.float64).reshape(-1, 7)
+        e = np.asarray(edges).reshape(-1, 2)
+        if e.size and (e.min() < 0 or e.max() > 0xFFFFFFFF):
+            raise capi.ArtpError(capi.ARTP_E_INVALID, "edge index outside the uint32 range")
+        e = np.ascontiguousarray(e, dtype=np.uint32)
+        nv, ne = s.shape[0], e.shape[0]
+        vf = np.empty(nv, np.uint8) if out_vertex is None else out_vertex
+        ef = np.empty(ne, np.uint8) if out_edge is None else out_edge
+        h.check(lib.artp_roadmap_updates(h.h, s.ctypes.data, nv, e.ctypes.data, ne, vf.ctypes.data, ef.ctypes.data))
+        return vf, ef
+
     def isValidBatchBits(self, states, out_valid, out_bits):
         """One shard step of the multi-GPU path: verdict bytes + bit-packed mask (CUDA float64 states), one call."""
         n = states.shape[0]

@@ -22,6 +22,7 @@
 #include "artp_tiles.cuh"
 #include "artp_sampler.cuh"
 #include "artp_basic.cuh"
+#include "artp_roadmap.cuh"
 
 namespace {
 
@@ -108,6 +109,13 @@ struct Handle {
   uint32_t* h_err = nullptr;        // host view
   uint32_t* d_err = nullptr;        // device view of the same word
   int tcap_override = 0;            // test hook (artp_debug_set_group_capacity)
+  // map change layer (artp_compute_change): the new map's `updated` layer, one bit per cell, and that map's geometry;
+  // the roadmap calls read both until the next artp_compute_change
+  uint32_t* d_chg_bits = nullptr;
+  size_t chg_words_cap = 0;
+  bool has_change = false;
+  int chg_rows = 0, chg_cols = 0;
+  double chg_res = 0, chg_cx = 0, chg_cy = 0;
   artp_stats stats{};
   std::string err;
   std::recursive_mutex mtx;   // recursive: host-buffer entry points hold it across their nested *_device call
@@ -414,6 +422,10 @@ int take_sticky_error(Handle* h) {
   if (h->h_err && *(volatile uint32_t*)h->h_err) {
     const uint32_t e = *(volatile uint32_t*)h->h_err;
     *(volatile uint32_t*)h->h_err = 0;
+    if (e & artp::kRoadmapBadEdge) {
+      h->err = "an edge referenced a vertex index >= nv (artp_roadmap_updates_device); its flag was set to 1";
+      return ARTP_E_INVALID;
+    }
     if (e & 2u) {
       h->err = "a box reached outside this handle's map window (artp_set_map_window: route samples to the shard that holds them, "
                "halo >= box half-diagonal + offsets); affected poses were marked invalid";
@@ -801,6 +813,7 @@ void artp_destroy(artp_handle* hh) {
   for (int k = 0; k < 2; ++k) for (int l = 0; l <= artp::kMaxLevel; ++l) { cudaFree(h->d_T[k][l]); cudaFree(h->d_NF[k][l]); }
   cudaFree(h->d_H[0]); cudaFree(h->d_H[1]); cudaFree(h->d_ctr); cudaFree(h->d_defer); cudaFree(h->d_stage);
   cudaFree(h->d_block_counts); cudaFree(h->d_recs); cudaFree(h->d_recs_f); cudaFree(h->d_recs_g); cudaFree(h->d_samp_layers); cudaFree(h->d_samp_scratch);
+  cudaFree(h->d_chg_bits);
   if (h->h_small_out) cudaFreeHost(h->h_small_out);
   if (h->h_err) cudaFreeHost(h->h_err);
   for (int g = 0; g < 2; ++g) if (h->chain_ev[g]) cudaEventDestroy(h->chain_ev[g]);
@@ -2102,6 +2115,179 @@ int artp_process_basic(artp_handle* hh, const float* elevation, const float* tra
   h->stats.kernel_launches += 11;
   h->stats.last_launches = 11;
   return ARTP_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Map change + roadmap reuse (artp_roadmap.cuh): processors::computeChange (change.cpp:9-51) and the per-vertex /
+// per-edge questions of LazyPRMStarMinUpdateMaintainer::update (lazy_prm_star_min_update.cpp:18-91, 123-135)
+// ---------------------------------------------------------------------------------------------------------------
+// grid_map::boundPositionToRange for one coordinate: epsilon = 10 * DBL_EPSILON, times |p| when |p| > 1.
+static void gm_bound(double* p, double L, double c) {
+  const double vto = 0.5 * L;
+  double s = (*p - c) + vto;
+  double eps = 10.0 * 2.220446049250313080847e-16;
+  if (std::fabs(*p) > 1.0) eps *= std::fabs(*p);
+  if (s <= 0.0) s = eps;
+  else if (s >= L) s = L - eps;
+  *p = (s + c) - vto;
+}
+
+// grid_map::SubmapGeometry(map, position, length) (getSubmapInformation): corners clamped into the map, converted to
+// indices; size = br - tl + 1; fails when the requested centre is outside the resulting submap (or a corner index is
+// outside the map, which only rounding can cause).
+static bool gm_submap(const artp_grid* m, double rx, double ry, double rlx, double rly, int start[2], int size[2]) {
+  const double Lx = m->rows * m->res, Ly = m->cols * m->res;
+  double tl[2] = {rx + 0.5 * rlx, ry + 0.5 * rly}, br[2] = {rx - 0.5 * rlx, ry - 0.5 * rly};
+  gm_bound(&tl[0], Lx, m->cx); gm_bound(&tl[1], Ly, m->cy);
+  gm_bound(&br[0], Lx, m->cx); gm_bound(&br[1], Ly, m->cy);
+  int ti, tj, bi, bj;
+  if (!artp::grid_index(m->rows, m->cols, m->res, m->cx, m->cy, tl[0], tl[1], ti, tj)) return false;
+  if (!artp::grid_index(m->rows, m->cols, m->res, m->cx, m->cy, br[0], br[1], bi, bj)) return false;
+  // getPositionFromIndex(top-left) + 0.5 res: the submap's corner
+  const double cx = ((m->cx + (0.5 * Lx - 0.5 * m->res)) + m->res * (-(double)ti)) + 0.5 * m->res;
+  const double cy = ((m->cy + (0.5 * Ly - 0.5 * m->res)) + m->res * (-(double)tj)) + 0.5 * m->res;
+  start[0] = ti; start[1] = tj;
+  size[0] = bi - ti + 1; size[1] = bj - tj + 1;
+  const double slx = size[0] * m->res, sly = size[1] * m->res;
+  const double spx = cx - 0.5 * slx, spy = cy - 0.5 * sly;
+  const double tx = -((rx - spx) - 0.5 * slx), ty = -((ry - spy) - 0.5 * sly);
+  return tx >= 0.0 && ty >= 0.0 && tx < slx && ty < sly;
+}
+
+static bool grid_ok(const artp_grid* m) {
+  return m && m->elevation && m->traversability_thresholded && m->rows > 0 && m->cols > 0 && m->res > 0.0 &&
+         (size_t)m->rows * (size_t)m->cols < ((size_t)1 << 31);
+}
+
+int artp_compute_change_device(artp_handle* hh, const artp_grid* map_new, const artp_grid* map_old,
+                               float height_change_for_update, float* d_updated, void* stream) {
+  if (!hh) return ARTP_E_INVALID;
+  Handle* h = reinterpret_cast<Handle*>(hh);
+  std::lock_guard<std::recursive_mutex> lk(h->mtx);
+  if (!grid_ok(map_new) || !grid_ok(map_old)) { h->err = "bad map (null layer, empty, res <= 0 or >= 2^31 cells)"; return ARTP_E_INVALID; }
+  CU_TRY(h, cudaSetDevice(h->device));
+  const cudaStream_t s = (cudaStream_t)stream;
+  ChainScope cs(h, 0, s);
+  if (cs.rc) return cs.rc;
+  const size_t ncell = (size_t)map_new->rows * map_new->cols, words = (ncell + 31) / 32;
+  if (h->chg_words_cap < words) {
+    CU_TRY(h, cudaDeviceSynchronize());   // growth only: earlier readers on any stream must be done
+    cudaFree(h->d_chg_bits);
+    h->d_chg_bits = nullptr; h->chg_words_cap = 0; h->has_change = false;
+    CU_TRY(h, cudaMalloc(&h->d_chg_bits, words * sizeof(uint32_t)));
+    h->chg_words_cap = words;
+  }
+  // change.cpp:15-25: both submap geometries, once, in double on the host
+  int sn[2], zn[2], so[2], zo[2];
+  const bool ok = gm_submap(map_new, map_old->cx, map_old->cy, map_old->rows * map_old->res, map_old->cols * map_old->res, sn, zn) &&
+                  gm_submap(map_old, map_new->cx, map_new->cy, map_new->rows * map_new->res, map_new->cols * map_new->res, so, zo);
+  artp::ChangeArgs a{};
+  a.e_new = map_new->elevation; a.t_new = map_new->traversability_thresholded;
+  a.e_old = map_old->elevation; a.t_old = map_old->traversability_thresholded;
+  a.rows_new = (uint32_t)map_new->rows; a.rows_old = (uint32_t)map_old->rows; a.ncell = (uint32_t)ncell;
+  if (ok) {
+    a.sn0 = sn[0]; a.sn1 = sn[1]; a.so0 = so[0]; a.so1 = so[1];
+    a.sx = std::min(zn[0], zo[0]); a.sy = std::min(zn[1], zo[1]);
+  }
+  a.thr = height_change_for_update;
+  a.bits = h->d_chg_bits;
+  a.upd = d_updated;
+  const unsigned grid = (unsigned)std::min<size_t>((ncell + 255) / 256, (size_t)h->sm_count * 16);
+  artp::change_kernel<<<grid, 256, 0, s>>>(a);
+  CU_TRY(h, cudaGetLastError());
+  h->has_change = true;
+  h->chg_rows = map_new->rows; h->chg_cols = map_new->cols;
+  h->chg_res = map_new->res; h->chg_cx = map_new->cx; h->chg_cy = map_new->cy;
+  h->stats.kernel_launches += 1;
+  h->stats.last_launches = 1;
+  return ARTP_OK;
+}
+
+int artp_compute_change(artp_handle* hh, const artp_grid* map_new, const artp_grid* map_old, float height_change_for_update,
+                        float* updated) {
+  if (!hh) return ARTP_E_INVALID;
+  Handle* h = reinterpret_cast<Handle*>(hh);
+  std::lock_guard<std::recursive_mutex> lk(h->mtx);   // held across stage -> launch -> D2H
+  if (!grid_ok(map_new) || !grid_ok(map_old)) { h->err = "bad map (null layer, empty, res <= 0 or >= 2^31 cells)"; return ARTP_E_INVALID; }
+  CU_TRY(h, cudaSetDevice(h->device));
+  int rc = chain_begin(h, 0, h->stream);
+  if (rc) return rc;
+  const size_t nn = (size_t)map_new->rows * map_new->cols, no = (size_t)map_old->rows * map_old->cols;
+  const size_t bn = (nn * sizeof(float) + 255) & ~(size_t)255, bo = (no * sizeof(float) + 255) & ~(size_t)255;
+  rc = ensure_stage(h, 3 * bn + 2 * bo);
+  if (rc) return rc;
+  char* st = (char*)h->d_stage;
+  artp_grid dn = *map_new, dold = *map_old;
+  dn.elevation = (const float*)st; dn.traversability_thresholded = (const float*)(st + bn);
+  dold.elevation = (const float*)(st + 2 * bn); dold.traversability_thresholded = (const float*)(st + 2 * bn + bo);
+  float* d_out = updated ? (float*)(st + 2 * bn + 2 * bo) : nullptr;
+  CU_TRY(h, cudaMemcpyAsync((void*)dn.elevation, map_new->elevation, nn * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+  CU_TRY(h, cudaMemcpyAsync((void*)dn.traversability_thresholded, map_new->traversability_thresholded, nn * sizeof(float),
+                            cudaMemcpyHostToDevice, h->stream));
+  CU_TRY(h, cudaMemcpyAsync((void*)dold.elevation, map_old->elevation, no * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+  CU_TRY(h, cudaMemcpyAsync((void*)dold.traversability_thresholded, map_old->traversability_thresholded, no * sizeof(float),
+                            cudaMemcpyHostToDevice, h->stream));
+  rc = artp_compute_change_device(hh, &dn, &dold, height_change_for_update, d_out, h->stream);
+  if (rc) return rc;
+  if (updated) CU_TRY(h, cudaMemcpyAsync(updated, d_out, nn * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+  CU_TRY(h, cudaStreamSynchronize(h->stream));
+  h->chain_busy[0] = false;
+  return ARTP_OK;
+}
+
+int artp_roadmap_updates_device(artp_handle* hh, const double* d_vertex_states, size_t nv, const uint32_t* d_edges, size_t ne,
+                                uint8_t* d_vertex_flags, uint8_t* d_edge_flags, void* stream) {
+  if (!hh) return ARTP_E_INVALID;
+  Handle* h = reinterpret_cast<Handle*>(hh);
+  std::lock_guard<std::recursive_mutex> lk(h->mtx);
+  if (!h->has_change) { h->err = "no change layer (artp_compute_change first)"; return ARTP_E_NOMAP; }
+  if ((nv && (!d_vertex_states || !d_vertex_flags)) || (ne && (!d_edges || !d_edge_flags))) { h->err = "null buffer"; return ARTP_E_INVALID; }
+  if (nv == 0 && ne == 0) return ARTP_OK;
+  CU_TRY(h, cudaSetDevice(h->device));
+  const cudaStream_t s = (cudaStream_t)stream;
+  ChainScope cs(h, 0, s);
+  if (cs.rc) return cs.rc;
+  const artp::RoadmapGeom g{h->d_chg_bits, h->chg_rows, h->chg_cols, h->chg_res, h->chg_cx, h->chg_cy};
+  const size_t threads = std::max(nv, ne * 32);
+  const unsigned grid = (unsigned)std::min<size_t>((threads + 255) / 256, (size_t)h->sm_count * 16);
+  artp::roadmap_kernel<<<grid, 256, 0, s>>>(g, d_vertex_states, nv, d_edges, ne, d_vertex_flags, d_edge_flags, h->d_err);
+  CU_TRY(h, cudaGetLastError());
+  h->stats.kernel_launches += 1;
+  h->stats.last_launches = 1;
+  return ARTP_OK;
+}
+
+int artp_roadmap_updates(artp_handle* hh, const double* vertex_states, size_t nv, const uint32_t* edges, size_t ne,
+                         uint8_t* vertex_flags, uint8_t* edge_flags) {
+  if (!hh) return ARTP_E_INVALID;
+  Handle* h = reinterpret_cast<Handle*>(hh);
+  std::lock_guard<std::recursive_mutex> lk(h->mtx);   // held across stage -> launch -> D2H
+  if (!h->has_change) { h->err = "no change layer (artp_compute_change first)"; return ARTP_E_NOMAP; }
+  if ((nv && (!vertex_states || !vertex_flags)) || (ne && (!edges || !edge_flags))) { h->err = "null buffer"; return ARTP_E_INVALID; }
+  for (size_t k = 0; k < 2 * ne; ++k)
+    if (edges[k] >= nv) { h->err = "edge " + std::to_string(k / 2) + " references a vertex index >= nv"; return ARTP_E_INVALID; }
+  if (nv == 0 && ne == 0) return ARTP_OK;
+  CU_TRY(h, cudaSetDevice(h->device));
+  int rc = chain_begin(h, 0, h->stream);
+  if (rc) return rc;
+  const size_t bs = (nv * 7 * sizeof(double) + 255) & ~(size_t)255, be = (ne * 2 * sizeof(uint32_t) + 255) & ~(size_t)255;
+  const size_t bv = (nv + 255) & ~(size_t)255;
+  rc = ensure_stage(h, bs + be + bv + ne);
+  if (rc) return rc;
+  char* st = (char*)h->d_stage;
+  double* d_s = (double*)st;
+  uint32_t* d_e = (uint32_t*)(st + bs);
+  uint8_t* d_vf = (uint8_t*)(st + bs + be);
+  uint8_t* d_ef = d_vf + bv;
+  if (nv) CU_TRY(h, cudaMemcpyAsync(d_s, vertex_states, nv * 7 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+  if (ne) CU_TRY(h, cudaMemcpyAsync(d_e, edges, ne * 2 * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
+  rc = artp_roadmap_updates_device(hh, d_s, nv, d_e, ne, d_vf, d_ef, h->stream);
+  if (rc) return rc;
+  if (nv) CU_TRY(h, cudaMemcpyAsync(vertex_flags, d_vf, nv, cudaMemcpyDeviceToHost, h->stream));
+  if (ne) CU_TRY(h, cudaMemcpyAsync(edge_flags, d_ef, ne, cudaMemcpyDeviceToHost, h->stream));
+  CU_TRY(h, cudaStreamSynchronize(h->stream));
+  h->chain_busy[0] = false;
+  return take_sticky_error(h);
 }
 
 size_t artp_cost_weights_size(void) { return artp_cnn::blob_floats(); }

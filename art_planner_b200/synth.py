@@ -86,6 +86,7 @@ class SynthMap:
     cx: float
     cy: float
     desc: str
+    traversability_thresholded: np.ndarray | None = None   # float32 0 / 1, Fortran order (make_map_pair)
 
     @property
     def rows(self) -> int:
@@ -376,3 +377,128 @@ def make_traversability(m: SynthMap, seed: int = 13):
     t = np.where(hash_uniform(seed, 42, blk) < 0.03, 0.05, t)                    # dead blobs
     obs = (hash_uniform(seed, 43, (np.arange(m.rows)[:, None] // 23) * 4096 + (np.arange(m.cols)[None, :] // 29)) > 0.06)
     return (np.asfortranarray(np.clip(t, 0.0, 1.0).astype(np.float32)), np.asfortranarray(obs.astype(np.float32)))
+
+
+# ---------------------------------------------------------------------------------------------
+# map updates: the old / new map pair processors::computeChange compares (change.cpp:9-51) and a roadmap on it
+# ---------------------------------------------------------------------------------------------
+def _world_map(seed: int, rows: int, cols: int, res: float, cx: float, cy: float, octaves: int) -> SynthMap:
+    """A view of the fBm world of `seed` centred at (cx, cy): elevation and a 0 / 1 traversability, both functions of
+    the cell centre's world position only, so two views agree wherever their cell centres coincide."""
+    m = SynthMap(np.zeros((rows, cols), np.float32, order="F"), np.zeros((1, 1), np.float32), res, cx, cy, "")
+    x, y = m.cell_xy()
+    e = fbm_height(seed, x[:, None], y[None, :], 0.6, 8.0, octaves).astype(np.float32)
+    t = (fbm_height(seed + 1, x[:, None], y[None, :], 1.0, 3.0, 2) > -0.35).astype(np.float32)
+    m.elevation = np.asfortranarray(e)
+    m.traversability_thresholded = np.asfortranarray(t)
+    return m
+
+
+def _blob_mask(m: SynthMap, bx: float, by: float, half: float):
+    """The cells whose centre is within `half` of (bx, by) along both axes, as a (row slice, column slice)."""
+    x, y = m.cell_xy()
+    ri, ci = np.nonzero(np.abs(x - bx) < half)[0], np.nonzero(np.abs(y - by) < half)[0]
+    if not ri.size or not ci.size:
+        return slice(0, 0), slice(0, 0)
+    return slice(ri[0], ri[-1] + 1), slice(ci[0], ci[-1] + 1)
+
+
+def make_map_pair(seed: int = 0, index: int = 0, rows: int = 1000, cols: int = 1000, res: float = 0.04,
+                  old_rows: int | None = None, old_cols: int | None = None, shift=None, thr: float = 0.1,
+                  n_blobs: int = 12, octaves: int = 4):
+    """(map_new, map_old) for processors::computeChange: two views of one fBm world, the old one centred at the origin,
+    the new one at `shift` (default: a non-integer number of cells, 5-15 % of the map length per axis, drawn from
+    (seed, index)), plus seeded changes in the new view -- height blobs above `thr`, below it and exactly at it (flat 0
+    in the old view, flat float32(thr) in the new one: |difference| == thr), NaN patches in either view, a -inf patch,
+    and traversability switched 1 -> 0 and 0 -> 1. Pure function of its arguments. Layers float32, Fortran order;
+    elevation_masked = elevation where traversable and finite, -inf elsewhere."""
+    old_rows = rows if old_rows is None else old_rows
+    old_cols = cols if old_cols is None else old_cols
+    u = hash_uniform(seed, 5000 + 16 * index, np.arange(4))
+    if shift is None:
+        lx, ly = rows * res, cols * res
+        sx = (0.05 + 0.10 * u[0]) * lx * (1 if u[2] < 0.5 else -1)
+        sy = (0.05 + 0.10 * u[1]) * ly * (1 if u[3] < 0.5 else -1)
+        shift = (sx, sy)
+    old = _world_map(seed, old_rows, old_cols, res, 0.0, 0.0, octaves)
+    new = _world_map(seed, rows, cols, res, float(shift[0]), float(shift[1]), octaves)
+    # blob centres inside the overlap of the two views
+    lo_x = max(old.cx - 0.5 * old.length[0], new.cx - 0.5 * new.length[0])
+    hi_x = min(old.cx + 0.5 * old.length[0], new.cx + 0.5 * new.length[0])
+    lo_y = max(old.cy - 0.5 * old.length[1], new.cy - 0.5 * new.length[1])
+    hi_y = min(old.cy + 0.5 * old.length[1], new.cy + 0.5 * new.length[1])
+    k = np.arange(8 * n_blobs)
+    bx = lo_x + (hi_x - lo_x) * hash_uniform(seed, 5001 + 16 * index, k)
+    by = lo_y + (hi_y - lo_y) * hash_uniform(seed, 5002 + 16 * index, k)
+    half = 0.1 + 0.4 * hash_uniform(seed, 5003 + 16 * index, k)
+    amt = hash_uniform(seed, 5004 + 16 * index, k)
+    e_new, e_old = new.elevation, old.elevation
+    t_new, t_old = new.traversability_thresholded, old.traversability_thresholded
+    thr32 = np.float32(thr)
+    for b in range(8 * n_blobs):
+        kind = b % 8
+        mn, mo = _blob_mask(new, bx[b], by[b], half[b]), _blob_mask(old, bx[b], by[b], half[b])
+        if kind == 0:                      # above the threshold
+            e_new[mn] += np.float32(thr * (1.05 + 2.0 * amt[b]))
+        elif kind == 1:                    # below it
+            e_new[mn] += np.float32(thr * 0.9 * amt[b])
+        elif kind == 2:                    # exactly at it
+            e_old[mo] = 0.0
+            e_new[mn] = thr32
+        elif kind == 3:                    # NaN in the new view
+            e_new[mn] = np.nan
+        elif kind == 4:                    # NaN in the old view
+            e_old[mo] = np.nan
+        elif kind == 5:                    # traversable -> untraversable
+            t_old[mo] = 1.0
+            t_new[mn] = 0.0
+        elif kind == 6:                    # untraversable -> traversable
+            t_old[mo] = 0.0
+            t_new[mn] = 1.0
+        else:                              # -inf (a hole) in the new view
+            e_new[mn] = -np.inf if amt[b] < 0.5 else np.inf
+    for m in (new, old):
+        m.elevation_masked = np.asfortranarray(
+            np.where((m.traversability_thresholded > 0.5) & np.isfinite(m.elevation), m.elevation, -np.inf).astype(np.float32))
+        m.desc = f"map pair seed={seed} index={index} view {m.rows}x{m.cols}@{res} centre=({m.cx:.4f}, {m.cy:.4f})"
+    return new, old
+
+
+def make_roadmap(m: SynthMap, n_vertices: int, n_edges: int, seed: int = 0, max_dist: float = 1.5, margin: float = 0.0):
+    """A PRM-like roadmap: n_vertices SE(3) states uniform over the map's extent grown by `margin` m on every side (so
+    some fall outside), and n_edges (source, target) index pairs among the vertex pairs closer than max_dist, found by
+    grid binning; which pairs and which direction each edge has are drawn from `seed`. Returns (states [nv, 7] float64,
+    edges [ne, 2] uint32); fewer edges when fewer pairs exist."""
+    k = np.arange(n_vertices)
+    lx, ly = m.length
+    x = m.cx - 0.5 * lx - margin + (lx + 2 * margin) * hash_uniform(seed, 6001, k)
+    y = m.cy - 0.5 * ly - margin + (ly + 2 * margin) * hash_uniform(seed, 6002, k)
+    states = np.zeros((n_vertices, 7), np.float64)
+    states[:, 0], states[:, 1], states[:, 6] = x, y, 1.0
+    bx = np.floor((x - x.min()) / max_dist).astype(np.int64)
+    by = np.floor((y - y.min()) / max_dist).astype(np.int64)
+    nbx, nby = int(bx.max()) + 3, int(by.max()) + 3
+    bid = (bx + 1) * nby + (by + 1)                     # one empty ring of bins around the occupied ones
+    order = np.argsort(bid, kind="stable")
+    cnt = np.bincount(bid, minlength=nbx * nby)
+    first = np.concatenate([[0], np.cumsum(cnt)[:-1]])
+    src_all, dst_all = [], []
+    for dx in (-1, 0, 1):
+        for dy in (-1, 0, 1):
+            nb = bid + dx * nby + dy
+            c = cnt[nb]
+            src = np.repeat(k, c)
+            off = np.arange(int(c.sum())) - np.repeat(np.cumsum(c) - c, c)
+            dst = order[np.repeat(first[nb], c) + off]
+            keep = src < dst
+            src, dst = src[keep], dst[keep]
+            d2 = (x[src] - x[dst]) ** 2 + (y[src] - y[dst]) ** 2
+            keep = d2 < max_dist * max_dist
+            src_all.append(src[keep]); dst_all.append(dst[keep])
+    src, dst = np.concatenate(src_all), np.concatenate(dst_all)
+    code = src.astype(np.uint64) * np.uint64(n_vertices) + dst.astype(np.uint64)
+    pick = np.argsort(hash_u64(seed, 6003, code), kind="stable")[:n_edges]
+    src, dst, code = src[pick], dst[pick], code[pick]
+    flip = (hash_u64(seed, 6004, code) & np.uint64(1)).astype(bool)
+    edges = np.stack([np.where(flip, dst, src), np.where(flip, src, dst)], axis=1).astype(np.uint32)
+    return states, np.ascontiguousarray(edges)

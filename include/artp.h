@@ -39,6 +39,14 @@
  *                                   art_planner_motion_cost/scripts/cost_query_server.py:145-169,
  *                                   predictor/predictor.py:28-44, predictor/cost_query.py:39-69)
  *   artp_combine_cost               MotionCostObjective::getCost / isFeasible (motion_cost_objective.h:54-66)
+ *   artp_compute_change[_device]    processors::computeChange (src/map/processors/change.cpp:9-51), the old-map processor
+ *                                   Planner::setUpMapProcessors installs when invalidate_updated_graph_components is set
+ *                                   (planner.cpp:60-69)
+ *   artp_roadmap_updates[_device]   the per-vertex / per-edge questions of LazyPRMStarMinUpdateMaintainer::update
+ *                                   (lazy_prm_star_min_update.cpp:123-135): isOutOfBounds for removeOutdatedVertices
+ *                                   (:58-72, :94-98) and wasUpdated(v) / wasUpdated(e) for invalidateUpdatedGraphComponents
+ *                                   (:18-54, :76-91) = Map::getUpdatedAtPosition / getUpdatedOnLine (map.h:86-89,
+ *                                   map.cpp:44-53)
  */
 #ifndef ARTP_H
 #define ARTP_H
@@ -243,7 +251,8 @@ int artp_get_stats(artp_handle* h, artp_stats* out);
  * artp_set_map from the box diagonals; cannot happen for boxes that passed artp_set_map unless the test hook below is
  * used) the affected pose / edge is reported INVALID (fail closed) and a sticky error is raised: host-buffer calls return
  * ARTP_E_LIMIT from the call that caused it; after asynchronous *_device calls, synchronise the stream and call
- * artp_poll_error (returns ARTP_E_LIMIT once, then clears). artp_get_stats reports it too. */
+ * artp_poll_error (returns ARTP_E_LIMIT once, then clears). artp_get_stats reports it too. artp_roadmap_updates_device
+ * raises the same sticky error for an edge index >= nv; it is reported as ARTP_E_INVALID. */
 int artp_poll_error(artp_handle* h);
 /* Test hook: cap the plane store at max_triangles (0 = no cap) from the next artp_set_map on. */
 int artp_debug_set_group_capacity(artp_handle* h, int max_triangles);
@@ -325,6 +334,37 @@ int artp_combine_cost(artp_handle* h, const float* cost3, size_t n, double* cost
 int artp_get_features(artp_handle* h, float* out, size_t n_floats, int* hf, int* wf);
 int artp_set_cnn_mode(artp_handle* h, int mode);
 int artp_get_cnn_timing(artp_handle* h, float* ms3);
+
+/* ---- processors::computeChange + LazyPRMStarMinUpdateMaintainer::update (roadmap reuse across replans) -----------
+ * grid_map_core is not in the reference tree, so its SubmapGeometry, index <-> position maps and LineIterator are used in
+ * the written form DESIGN.md section 4.6 gives (buffer start index (0,0)); results are exact (float compares and integer
+ * grid walks). */
+typedef struct artp_grid {            /* one map's geometry + the two layers computeChange reads */
+  const float* elevation;             /* grid_map layout, rows x cols column-major; NaN / inf allowed */
+  const float* traversability_thresholded;
+  int rows, cols; double res, cx, cy;
+} artp_grid;
+/* computeChange(map_new, map_old, height_change_for_update) (change.cpp:9-51): `updated` of the new map is 1 except over
+ * the overlap of SubmapGeometry(new, old.position, old.length) and SubmapGeometry(old, new.position, new.length), where a
+ * cell is 0 unless |e_new - e_old| > thr or t_old - t_new > 0.5 (float; NaN compares false). Either submap failing
+ * leaves all ones. The layer stays on the handle, one bit per cell, with the new map's geometry, until the next
+ * artp_compute_change; `updated` (nullable) receives it as floats (exact 0 / 1) in the new map's layout. HOST layers. */
+int artp_compute_change(artp_handle* h, const artp_grid* map_new, const artp_grid* map_old,
+                        float height_change_for_update, float* updated);
+/* Same with DEVICE layers on `stream`, asynchronous; d_updated nullable. */
+int artp_compute_change_device(artp_handle* h, const artp_grid* map_new, const artp_grid* map_old,
+                               float height_change_for_update, float* d_updated, void* stream);
+/* Against the last change layer (ARTP_E_NOMAP before the first artp_compute_change; artp_set_map is not needed):
+ * vertex_flags[v]: 0 keep, 1 updated (-> VALIDITY_UNKNOWN), 2 outside the new map (removeOutdatedVertices), from x, y of
+ * vertex_states (nv x 7 doubles, x y z qx qy qz qw);
+ * edge_flags[e] for edges[e] = (source, target) vertex indices: 0, 1 a cell of grid_map's LineIterator from source to
+ * target is updated, 2 an endpoint is outside (the edge goes with its vertex and is never walked).
+ * Every edge index must be < nv: the host entry returns ARTP_E_INVALID before launching anything; the device entry
+ * fails closed (flag 1) and raises the sticky error that artp_poll_error reports as ARTP_E_INVALID. */
+int artp_roadmap_updates(artp_handle* h, const double* vertex_states, size_t nv,
+                         const uint32_t* edges, size_t ne, uint8_t* vertex_flags, uint8_t* edge_flags);
+int artp_roadmap_updates_device(artp_handle* h, const double* d_vertex_states, size_t nv, const uint32_t* d_edges,
+                                size_t ne, uint8_t* d_vertex_flags, uint8_t* d_edge_flags, void* stream);
 
 /* Version string of the library / kernel image ("artp <ver> sm_100a"). */
 const char* artp_version(void);

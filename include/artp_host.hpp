@@ -7,6 +7,9 @@
 //                                        lazy_prm_star_min_update.cpp:725)
 //   art_planner::PathLengthObjective    include/art_planner/objectives/path_length_objective.h, .cpp:26-70
 //   art_planner::MotionCostObjective    include/art_planner/objectives/motion_cost_objective.h:19-78, .cpp:28-95
+//   processors::computeChange           src/map/processors/change.cpp:9-51 (+ Map::getUpdatedAtPosition, map.h:86-89)
+//   LazyPRMStarMinUpdateMaintainer      src/planners/lazy_prm_star_min_update.cpp:18-91, 123-135 (flags only; the Boost
+//                                        graph surgery stays with the planner)
 // OMPL / Eigen / grid_map are not available in this build image, so the classes are written against three tiny
 // stand-ins (State = the seven doubles utils.h:25-38 reads from an SE3StateSpace::StateType, Map = two column-major
 // float layers + geometry as grid_map stores them, EdgeMatrix = row-major float matrix). With -DARTP_WITH_OMPL the
@@ -64,6 +67,26 @@ struct Map {
   // layers the sampler reads (Map::getNormal / getPlaneFitStdDev map.h:94-116, probability_distribution.cpp:20-46);
   // cum_prob_rowwise = column 0 of "cum_prob_rowwise_hack". Empty when no sampler is used.
   std::vector<float> normal_x, normal_y, normal_z, plane_fit_std_dev, cum_prob, cum_prob_rowwise;
+  // processors::Basic's "traversability_thresholded" (0 / 1) and computeChange's "updated" (change.cpp:50).
+  std::vector<float> traversability_thresholded, updated;
+
+  // grid_map getIndexFromPosition + checkIfPositionWithinMap (buffer start index (0,0)); false outside the map (an index
+  // past the last cell from rounding counts as outside, DESIGN 4.6).
+  bool getIndex(double x, double y, int* row, int* col) const {
+    const double lx = rows * resolution, ly = cols * resolution;
+    const double tx = -((x - position_x) - 0.5 * lx), ty = -((y - position_y) - 0.5 * ly);
+    if (!(tx >= 0.0 && ty >= 0.0 && tx < lx && ty < ly)) return false;
+    *row = static_cast<int>(-(((x - 0.5 * lx) - position_x) / resolution));
+    *col = static_cast<int>(-(((y - 0.5 * ly) - position_y) / resolution));
+    return *row >= 0 && *col >= 0 && *row < rows && *col < cols;
+  }
+  bool isInside(double x, double y) const { int r, c; return getIndex(x, y, &r, &c); }
+  // Map::getUpdatedAtPosition (map.h:86-89): throws std::out_of_range outside the map, as GridMap::atPosition does.
+  bool getUpdatedAtPosition(double x, double y) const {
+    int r, c;
+    if (!getIndex(x, y, &r, &c)) throw std::out_of_range("getUpdatedAtPosition: position outside the map");
+    return updated.at(static_cast<size_t>(r) + static_cast<size_t>(c) * rows) > std::numeric_limits<float>::epsilon();
+  }
 };
 
 inline artp_params toArtp(const Params& p) {
@@ -480,6 +503,68 @@ class MotionCostObjective {
  private:
   StateValidityCheckerPtr checker_;
   std::unique_ptr<MotionCostFunc> motion_cost_func_;
+};
+
+namespace processors {
+// processors::computeChange (change.cpp:9-51) on the device: fills map_new->updated (1 where the height changed by more
+// than height_change_for_update or the traversability went 1 -> 0 over the overlap of the two maps, and everywhere
+// outside it). The layer also stays on the handle, bit-packed, for LazyPRMStarMinUpdateMaintainer.
+inline void computeChange(const HandlePtr& handle, const std::shared_ptr<Map>& map_new, const std::shared_ptr<Map>& map_old,
+                          float height_change_for_update) {
+  auto grid = [](const Map& m, const char* which) {
+    const size_t ncell = static_cast<size_t>(m.rows) * m.cols;
+    if (m.elevation.size() != ncell || m.traversability_thresholded.size() != ncell)
+      throw std::invalid_argument(std::string("computeChange: ") + which + " map needs elevation and traversability_thresholded");
+    artp_grid g{};
+    g.elevation = m.elevation.data(); g.traversability_thresholded = m.traversability_thresholded.data();
+    g.rows = m.rows; g.cols = m.cols; g.res = m.resolution; g.cx = m.position_x; g.cy = m.position_y;
+    return g;
+  };
+  const artp_grid gn = grid(*map_new, "new"), go = grid(*map_old, "old");
+  map_new->updated.resize(static_cast<size_t>(map_new->rows) * map_new->cols);
+  handle->check(artp_compute_change(handle->get(), &gn, &go, height_change_for_update, map_new->updated.data()),
+                "artp_compute_change");
+}
+}  // namespace processors
+
+// LazyPRMStarMinUpdateMaintainer::update (lazy_prm_star_min_update.cpp:123-135) for a roadmap given as arrays, against
+// the change layer of the last processors::computeChange on the same handle. The per-vertex / per-edge questions run in
+// one device call; the Boost graph surgery (removeVertices, components, start / goal re-insertion) stays with the planner.
+class LazyPRMStarMinUpdateMaintainer {
+ public:
+  static constexpr unsigned int VALIDITY_UNKNOWN = 0, VALIDITY_TRUE = 1;   // ompl::geometric::LazyPRM's flags
+  explicit LazyPRMStarMinUpdateMaintainer(const HandlePtr& handle) : handle_(handle) {}
+
+  // edges: 2 vertex indices per edge (boost::source, boost::target). Returns the vertices removeOutdatedVertices
+  // (:58-72) removes -- those outside the new map -- in ascending order; their edges go with them. Then, when
+  // invalidate_updated_graph_components is set, invalidateUpdatedGraphComponents (:18-54) on what stays: every
+  // VALIDITY_TRUE vertex on an updated cell and every VALIDITY_TRUE edge whose grid line crosses one becomes
+  // VALIDITY_UNKNOWN. Other flags are left as they are.
+  std::vector<size_t> update(const std::vector<State>& vertices, std::vector<unsigned int>* vertex_validity,
+                             const std::vector<uint32_t>& edges, std::vector<unsigned int>* edge_validity,
+                             bool invalidate_updated_graph_components = true) const {
+    const size_t nv = vertices.size(), ne = edges.size() / 2;
+    if (edges.size() % 2 || vertex_validity->size() != nv || edge_validity->size() != ne)
+      throw std::invalid_argument("LazyPRMStarMinUpdateMaintainer::update: size mismatch");
+    std::vector<uint8_t> vf(nv), ef(ne);
+    handle_->check(artp_roadmap_updates(handle_->get(), nv ? &vertices[0].x : nullptr, nv, ne ? edges.data() : nullptr, ne,
+                                        vf.data(), ef.data()), "artp_roadmap_updates");
+    std::vector<size_t> removed;
+    for (size_t v = 0; v < nv; ++v) {
+      if (vf[v] == 2) { removed.push_back(v); continue; }
+      unsigned int& vd = (*vertex_validity)[v];
+      if (invalidate_updated_graph_components && (vd & VALIDITY_TRUE) && vf[v] == 1) vd = VALIDITY_UNKNOWN;
+    }
+    if (invalidate_updated_graph_components)
+      for (size_t e = 0; e < ne; ++e) {
+        unsigned int& ed = (*edge_validity)[e];
+        if ((ed & VALIDITY_TRUE) && ef[e] == 1) ed = VALIDITY_UNKNOWN;
+      }
+    return removed;
+  }
+
+ private:
+  HandlePtr handle_;
 };
 
 }  // namespace artp_host
